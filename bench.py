@@ -54,6 +54,9 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the side measurements of the other BASELINE configs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (image features, last-position "
+                         "prefill logits, generated token ids) as DIR/<name>.npy, at most 64 MB in all")
     return ap.parse_args()
 
 
@@ -340,9 +343,10 @@ def synth_host_inputs(B, Lt, seed):
 
 
 def measure_device_resident(engine, m, B, S, N, steps, warmup, seed=1, fp8=False, world=1, dev=None, sampler=None,
-                            isolate_decode=False):
+                            isolate_decode=False, return_outputs=False):
     """One workload through the C-ABI with every input already in HBM: encode_images -> splice -> prefill -> N-1 greedy decode
-    steps, timed with CUDA events on the launching stream. Returns per-stage ms (max over ranks) and derived rates."""
+    steps, timed with CUDA events on the launching stream. Returns per-stage ms (max over ranks) and derived rates, and with
+    `return_outputs` the last timed step's results as host tensors."""
     import numpy as np
     from llava import _b2
     from llava._b2 import replicas
@@ -370,6 +374,7 @@ def measure_device_resident(engine, m, B, S, N, steps, warmup, seed=1, fp8=False
         if N > 1:
             engine.decode_greedy(kv, first, N - 1, out=out_tokens)
         if ev: ev[3].record()
+        return feats, logits, first
 
     for _ in range(warmup):
         device_step()
@@ -383,10 +388,15 @@ def measure_device_resident(engine, m, B, S, N, steps, warmup, seed=1, fp8=False
     evs = [[torch.cuda.Event(enable_timing=True) for _ in range(4)] for _ in range(steps)]
     launches0 = _b2.launch_count()
     for i in range(steps):
-        device_step(evs[i])
+        last = device_step(evs[i])
     torch.cuda.synchronize()
     launches = _b2.launch_count() - launches0
     clocks = sampler.stop() if sampler is not None else None
+    outputs = None
+    if return_outputs:
+        feats, logits, first = last
+        outputs = {"tokens": torch.cat([first[None], out_tokens[:N - 1]]).t().double().cpu(),
+                   "prefill_logits": logits.float().cpu(), "image_features": feats.float().cpu()}
     t_enc = sum(e[0].elapsed_time(e[1]) for e in evs) / steps
     t_pre = sum(e[1].elapsed_time(e[2]) for e in evs) / steps
     t_dec = sum(e[2].elapsed_time(e[3]) for e in evs) / steps
@@ -419,11 +429,35 @@ def measure_device_resident(engine, m, B, S, N, steps, warmup, seed=1, fp8=False
     dec_ms = t_dec / steps_dec
     return dict(t_total=t_total, t_enc=t_enc, t_pre=t_pre, t_dec=t_dec, dec_step_ms=dec_ms, launches=launches, clocks=clocks,
                 dec_step_ms_isolated=dec_iso,
-                work=work, out_tokens=out_tokens, images_host=images_host, ids_host=ids_host,
+                work=work, out_tokens=out_tokens, images_host=images_host, ids_host=ids_host, outputs=outputs,
                 decode_gbs=work["decode_bytes_per_step"] / (dec_ms * 1e-3) / 1e9,
                 decode_frac=work["decode_bytes_per_step"] / (dec_ms * 1e-3) / 1e9 / hbm_peak,
                 prefill_tflops=work["prefill_flops"] / (t_pre * 1e-3) / 1e12,
                 encode_tflops=work["encode_flops"] / (t_enc * 1e-3) / 1e12)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, outputs):
+    """Writes each host tensor as <path>/<name>.npy (float64 token ids, float32 otherwise). An array that does not fit in
+    what is left of DUMP_BYTES keeps a fixed, seeded sample of its rows (last dimension kept whole); the sampled row
+    indices go to <name>_rows.npy."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_BYTES
+    for name, t in outputs.items():
+        a = t.numpy()
+        if a.nbytes > left:
+            rows = a.reshape(-1, a.shape[-1])
+            k = max(1, left // (rows.shape[1] * a.itemsize + 8) - 1)
+            idx = np.sort(np.random.default_rng(0).choice(rows.shape[0], size=k, replace=False))
+            a = rows[idx]
+            np.save(os.path.join(path, f"{name}_rows.npy"), idx.astype(np.float64))
+            left -= idx.size * 8 + 128
+        np.save(os.path.join(path, f"{name}.npy"), a)
+        left -= a.nbytes + 128  # .npy header
 
 
 def config_line(name, m, B, S, N, r, fp8=False):
@@ -634,7 +668,10 @@ def run_ours(args):
     with torch.cuda.stream(stream), torch.no_grad():
         # ---------------- device-resident arm ----------------
         r = measure_device_resident(engine, m, B, S, N, args.steps, args.warmup, seed=1 + rank, fp8=args.fp8, world=world,
-                                    dev=dev, sampler=ClockSampler(local) if rank == 0 else None)
+                                    dev=dev, sampler=ClockSampler(local) if rank == 0 else None,
+                                    return_outputs=bool(args.dump_outputs) and rank == 0)
+        if r["outputs"] is not None:
+            dump_outputs(args.dump_outputs, r.pop("outputs"))
         images_host, ids_host, out_tokens = r["images_host"], r["ids_host"], r["out_tokens"]
         tokens_per_step = world * B * (S + N)
         value = tokens_per_step / (r["t_total"] * 1e-3)
